@@ -2,6 +2,7 @@
 """bench.py - the measurement contract of this repo.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c3f32|c4|c5|c1] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input: the FULL stats_generator
 (measures_of_counts / centralTendency / cardinality / dispersion / percentiles / shape) of a synthetic frame that is
@@ -17,6 +18,7 @@ oracle on the bit-identical NumPy twin of the generator (outside the timed regio
 oracle restatement on the host cores (Spark is not available on the box).
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -102,8 +104,14 @@ class ClockSampler:
             self.f = open(self.path, "w")
             self.proc = subprocess.Popen(["nvidia-smi", "--query-gpu=" + self.Q, "--format=csv,noheader,nounits",
                                           "-lms", str(self.period_ms), "-i", str(self.gpu)], stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self._kill)      # a run that fails before stop() must not leave the sampler polling
         except Exception:
             self.proc = None
+
+    def _kill(self):
+        if self.proc is not None and self.proc.poll() is None:
+            self.proc.kill()
+            self.proc.wait()
 
     def begin(self):
         """Open the sampling window (call right before the timed region; starts the sampler if start() was not called)."""
@@ -168,7 +176,7 @@ class ClockSampler:
 # ---------------------------------------------------------------------------------------------
 
 def stats_step(frame, keep_cache=False):
-    """Full stats_generator through the public API; returns the result frames (pandas)."""
+    """Full stats_generator through the public API; returns the result frames (pandas), in STATS_FUNCTIONS order."""
     import anovos.data_analyzer.stats_generator as sg
     if not keep_cache:
         frame._cache = {k: v for k, v in frame._cache.items() if isinstance(k, tuple) and k and k[0] == "desc"}
@@ -176,6 +184,62 @@ def stats_step(frame, keep_cache=False):
            sg.measures_of_cardinality(None, frame), sg.measures_of_dispersion(None, frame),
            sg.measures_of_percentiles(None, frame), sg.measures_of_shape(None, frame)]
     return [o.toPandas() for o in out]
+
+
+STATS_FUNCTIONS = ["measures_of_counts", "measures_of_centralTendency", "measures_of_cardinality", "measures_of_dispersion",
+                   "measures_of_percentiles", "measures_of_shape"]
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, named_frames, limit_bytes=DUMP_LIMIT_BYTES):
+    """Write the result tables of the last timed step as `path/<table>.<field>.npy`, float64, one value per row in the order the
+    caller receives the rows.  Every value written is finite: where a field holds a cell that is null or not finite, that cell
+    is 0 in `<table>.<field>.npy` and `<table>.<field>.nonfinite.npy` says what the caller gets there (0 = the value written,
+    1 = null / NaN, 2 = +inf, 3 = -inf).  A text field (the attribute name, the mode) is written as the CRC-32 of its UTF-8
+    text in `<table>.<field>.crc32.npy`, and also parsed as a number in `<table>.<field>.npy` when some cell holds one (the
+    mode of a numeric column; text that is not a number counts as null there).  When the arrays would exceed `limit_bytes`,
+    every table keeps the same share of its rows, picked by a generator with a fixed seed; the attribute CRCs name the rows
+    kept."""
+    import zlib
+    import numpy as np
+    import pandas as pd
+
+    def number(v):
+        try:
+            return float(v)      # exact, unlike pandas' fast text parser
+        except (TypeError, ValueError):
+            return np.nan
+    arrays = []
+
+    def add(name, field, a):
+        code = np.select([np.isnan(a), a == np.inf, a == -np.inf], [1.0, 2.0, 3.0], 0.0)
+        if code.any():
+            arrays.append((name, field + ".nonfinite", code))
+            a = np.where(code == 0, a, 0.0)
+        arrays.append((name, field, a))
+    for name, df in named_frames:
+        for field in df.columns:
+            s = df[field]
+            if pd.api.types.is_numeric_dtype(s) or pd.api.types.is_bool_dtype(s):
+                add(name, field, s.to_numpy(dtype=np.float64, na_value=np.nan))
+                continue
+            num = np.array([np.nan if pd.isna(v) else number(v) for v in s.tolist()], dtype=np.float64)
+            if not np.isnan(num).all():
+                add(name, field, num)
+            add(name, field + ".crc32", np.array([np.nan if pd.isna(v) else float(zlib.crc32(str(v).encode("utf-8")))
+                                                  for v in s.tolist()], dtype=np.float64))
+    total = sum(a.nbytes for _, _, a in arrays)
+    keep = {}
+    if total > limit_bytes:
+        share = limit_bytes / total
+        for name, df in named_frames:
+            n = len(df)
+            keep[name] = np.sort(np.random.default_rng(0).choice(n, int(n * share), replace=False))
+    os.makedirs(path, exist_ok=True)
+    for name, field, a in arrays:
+        np.save(os.path.join(path, "%s.%s.npy" % (name, field)), a[keep[name]] if name in keep else a)
 
 
 class StdoutGuard:
@@ -289,6 +353,8 @@ def _run_ours(args, out):
     e1.record()
     barrier()
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, list(zip(STATS_FUNCTIONS, last)))
     ms = e0.elapsed_time(e1)
     launches = engine.launch_count - l0
     kt = engine.timer.totals()
@@ -628,6 +694,8 @@ def _run_c1(args, out, wl, world, rank, local):
     e1.record()
     torch.cuda.synchronize()
     clk = clocks.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [("measures_of_centralTendency", res)])
     ms = e0.elapsed_time(e1)
     kt = engine.timer.totals()
     engine.timer = None
@@ -750,6 +818,9 @@ def _run_stream(args, out, wl, rows, cols, world, rank, local):
     e1.record()
     barrier()
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, list(zip(["drift_statistics", "source.measures_of_counts", "source.measures_of_shape",
+                                                  "target.measures_of_counts", "target.measures_of_shape"], res)))
     ms = e0.elapsed_time(e1)
     launches = engine.launch_count - l0
     kt = engine.timer.totals()
@@ -1151,7 +1222,13 @@ def main():
     ap.add_argument("--cols", type=int, default=0)
     ap.add_argument("--chunk", type=int, default=0, help="rows per chunk of the streamed workloads (c4, c5)")
     ap.add_argument("--no-extras", action="store_true", help="profiling runs: skip e2e / cpu_baseline / fused extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result tables of the last timed step to DIR/<table>.<field>.npy (rank 0; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
